@@ -9,6 +9,7 @@ metric = images+256-token generations per second (whole job, all GPUs).
   python bench.py --gpus 1 --steps 5 --warmup 3            # this repo's CUDA path
   python bench.py --impl reference ...                      # reference algorithm on the host cores (CPU oracle port)
   torchrun --nproc-per-node N bench.py --gpus N ...         # data parallel, one rank per GPU, weak scaling
+  python bench.py ... --dump-outputs DIR                    # also write the last timed step's tokens as DIR/tokens.npy
 """
 import argparse
 import json
@@ -43,7 +44,21 @@ def parse():
                     help="weak: --batch-per-gpu requests on every GPU; strong: a fixed global batch of 64 (SURVEY 8d config 4: B_local = 64/N)")
     ap.add_argument("--no-extras", action="store_true", help="skip the configs[2] / configs[4] / strong-scaling / HF-CUDA blocks of the default line")
     ap.add_argument("--pdl", type=int, default=int(os.environ.get("VCLA_PDL", "1")))
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="native arm: after the timed steps, write the (global batch, new tokens) greedy "
+                                                          "tokens of the last timed step to DIR/tokens.npy (float64), to compare builds")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the native arm's outputs; use it with --impl native")
+    return args
+
+
+def dump_outputs(out_dir, tokens):
+    """Write what one timed step returned to its caller: the greedy tokens, exact in float64."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "tokens.npy"), tokens.cpu().numpy().astype(np.float64))
 
 
 def peaks():
@@ -296,7 +311,7 @@ def run_config(args, world, rank, Bl, T, n_new, steps, warmup, with_e2e, with_tr
     with ClockSampler(int(os.environ.get("LOCAL_RANK", "0"))) as clocks:
         ms, out = timed(step_device, steps)
     res = {"B_local": Bl, "B": B, "T": T, "S": S, "n_new": n_new, "ms": ms, "steps": steps, "value": B * steps / (ms / 1000.0),
-           "launches": eng.kernel_launches(reset=True), "clocks": clocks.summary()}
+           "launches": eng.kernel_launches(reset=True), "clocks": clocks.summary(), "tokens": out}
     pre_ms = [a.elapsed_time(b) for a, b in zip(ev.get("start", []), ev.get("prefill_done", []))]
     dec_ms = [a.elapsed_time(b) for a, b in zip(ev.get("prefill_done", []), ev.get("done", []))]
     pk = peaks()
@@ -387,6 +402,8 @@ def run_native(args):
     Bl, n_new, T = args.batch_per_gpu, args.new_tokens, args.prompt_tokens
     B, S = Bl * world, T + NQ
     main = run_config(args, world, rank, Bl, T, n_new, args.steps, args.warmup, with_e2e=True, with_trace=True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, main["tokens"])
     pk = peaks()
     cfg_name = {(8, 64, 256): "1", (32, 128, 256): "2", (16, 1024, 512): "4"}.get((Bl, T, n_new), "*")
     line = {"metric": METRIC, "value": main["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
@@ -487,18 +504,14 @@ def run_native(args):
 # /root/reference is not on the GPU box, so the composite module is re-assembled from the very HF classes it calls
 # (modeling_visualcla.py:346-391) and the oracle's torch restatement of the in-repo Resampler, run on the device.
 # ----------------------------------------------------------------------------------------------------------------
-def run_hf_cuda(args, emit=True):
+def hf_cuda_step(B, T, n_new, dt):
+    """Build the HF composite on cuda:0 with random weights and return step(): one batch of greedy generations, (B, n_new) tokens."""
     import torch
     from transformers import LlamaConfig, LlamaForCausalLM, GenerationConfig
     from transformers.models.clip.modeling_clip import CLIPVisionConfig, CLIPVisionModel
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import visualcla_oracle as O
-    if int(os.environ.get("RANK", "0")) != 0:
-        return
-    dt = getattr(torch, args.hf_dtype)
-    B, n_new, T = args.batch_per_gpu, args.new_tokens, args.prompt_tokens
     cfg = O.PathConfig()
-    torch.cuda.set_device(0)
     old = torch.get_default_dtype()
     torch.set_default_dtype(dt)
     with torch.device("cuda"):
@@ -522,22 +535,32 @@ def run_hf_cuda(args, emit=True):
         x = torch.cat([emb[:, :2], img.to(dt), emb[:, 2:]], dim=1)
         mask = torch.ones(x.shape[:2], dtype=torch.long, device="cuda")
         return llama.generate(inputs_embeds=x, attention_mask=mask, generation_config=gc)
+    return step
 
-    for _ in range(max(1, min(args.warmup, 1))):
+
+def run_hf_cuda(args, emit=True):
+    """Time args.steps generations of the HF composite after max(1, args.warmup) warm-up generations (one is needed to check the shape)."""
+    import torch
+    if int(os.environ.get("RANK", "0")) != 0:
+        return
+    B, n_new, T = args.batch_per_gpu, args.new_tokens, args.prompt_tokens
+    torch.cuda.set_device(0)
+    step = hf_cuda_step(B, T, n_new, getattr(torch, args.hf_dtype))
+    warmup = max(1, args.warmup)
+    for _ in range(warmup):
         out = step()
     assert out.shape == (B, n_new), out.shape
     torch.cuda.synchronize()
-    k = max(1, min(args.steps, 3))
     t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t0.record()
-    for _ in range(k):
+    for _ in range(args.steps):
         step()
     t1.record()
     torch.cuda.synchronize()
-    ms = t0.elapsed_time(t1) / k
-    del llama, clip, w
+    ms = t0.elapsed_time(t1) / args.steps
+    del step, out
     torch.cuda.empty_cache()
-    line = ({"impl": "hf-cuda", "metric": METRIC, "value": B / (ms / 1e3), "unit": UNIT, "n_gpus": 1, "steps": k, "warmup": 1, "ms_per_step": ms,
+    line = ({"impl": "hf-cuda", "metric": METRIC, "value": B / (ms / 1e3), "unit": UNIT, "n_gpus": 1, "steps": args.steps, "warmup": warmup, "ms_per_step": ms,
                       "higher_is_better": True, "dtype": args.hf_dtype, "data": "synthetic, random weights",
                       "config": {"workload": f"batch {B}, {T}-token prompts + 64 image tokens, {n_new} greedy tokens; HF CLIPVisionModel + torch Resampler + "
                                              f"HF LlamaForCausalLM.generate(inputs_embeds) eager/SDPA, transformers {__import__('transformers').__version__}"}})

@@ -49,6 +49,88 @@ def test_native_arm_refuses_to_run_without_gpu():
     assert r.returncode != 0 and "no CPU fallback" in (r.stderr + r.stdout)
 
 
+def test_dump_outputs_and_its_arguments(bench, tmp_path, monkeypatch):
+    """--dump-outputs DIR writes the timed step's tokens exactly (float64) as DIR/tokens.npy; --steps below 1 is refused, and so is
+    --dump-outputs with any arm but the native one, before any work starts."""
+    import numpy as np
+    import torch
+    tok = torch.randint(0, 49958, (8, 256), generator=torch.Generator().manual_seed(0))
+    bench.dump_outputs(str(tmp_path / "out"), tok)
+    got = np.load(tmp_path / "out" / "tokens.npy")
+    assert got.dtype == np.float64 and got.shape == (8, 256) and np.array_equal(got, tok.numpy())
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "3", "--dump-outputs", str(tmp_path)])
+    assert bench.parse().steps == 3
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)], ["--impl", "hf-cuda", "--dump-outputs", str(tmp_path)]):
+        monkeypatch.setattr(sys, "argv", ["bench.py"] + argv)
+        with pytest.raises(SystemExit):
+            bench.parse()
+
+
+def test_native_arm_times_steps_and_dumps_that_runs_tokens(bench, tmp_path, monkeypatch, capsys):
+    """run_native hands --steps and --warmup to the timed configuration and dumps the tokens that timed run returned (the device stands
+    in as a fake run_config: no GPU here)."""
+    import numpy as np
+    import torch
+    from visualcla import _native
+    for k in ("WORLD_SIZE", "RANK", "LOCAL_RANK"):
+        monkeypatch.delenv(k, raising=False)
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: True)
+    monkeypatch.setattr(torch.cuda, "set_device", lambda *a: None)
+    monkeypatch.setattr(_native, "load", lambda: type("Lib", (), {"vcla_set_pdl": staticmethod(lambda on: None)})())
+    tok = torch.randint(0, 49958, (8, 256), generator=torch.Generator().manual_seed(1))
+    calls = []
+
+    def fake_run_config(args, world, rank, Bl, T, n_new, steps, warmup, with_e2e, with_trace):
+        calls.append((Bl, T, n_new, steps, warmup, with_e2e, with_trace))
+        return {"value": 1.0, "ms": 750.0 * steps, "steps": steps, "launches": 0, "clocks": {}, "e2e": {}, "tokens": tok}
+
+    monkeypatch.setattr(bench, "run_config", fake_run_config)
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "4", "--warmup", "2", "--no-extras", "--no-cpu-baseline",
+                                      "--dump-outputs", str(tmp_path / "dump")])
+    bench.run_native(bench.parse())
+    assert calls == [(8, 64, 256, 4, 2, True, True)]
+    line = json.loads(capsys.readouterr().out.strip().splitlines()[-1])
+    assert line["steps"] == 4 and line["ms_per_step"] == pytest.approx(750.0)
+    assert np.array_equal(np.load(tmp_path / "dump" / "tokens.npy"), tok.numpy())
+
+
+def test_hf_cuda_arm_times_exactly_steps(bench, monkeypatch):
+    """The informational HF arm times --steps generations after --warmup ones (at least one, to check the output shape)."""
+    import argparse
+    import torch
+    monkeypatch.delenv("RANK", raising=False)
+    calls = []
+
+    def fake_step_builder(B, T, n_new, dt):
+        def step():
+            calls.append(1)
+            return torch.zeros(B, n_new, dtype=torch.long)
+        return step
+
+    class FakeEvent:
+        def __init__(self, **k):
+            pass
+
+        def record(self):
+            pass
+
+        def elapsed_time(self, other):
+            return 700.0
+
+    monkeypatch.setattr(bench, "hf_cuda_step", fake_step_builder)
+    monkeypatch.setattr(torch.cuda, "Event", FakeEvent)
+    for f in ("set_device", "synchronize", "empty_cache"):
+        monkeypatch.setattr(torch.cuda, f, lambda *a: None)
+    for warmup, steps in ((2, 7), (0, 1), (5, 5)):
+        calls.clear()
+        ns = argparse.Namespace(hf_dtype="float16", batch_per_gpu=2, new_tokens=3, prompt_tokens=4, warmup=warmup, steps=steps)
+        line = bench.run_hf_cuda(ns, emit=False)
+        assert len(calls) == max(1, warmup) + steps
+        assert line["steps"] == steps and line["warmup"] == max(1, warmup) and line["ms_per_step"] == pytest.approx(700.0 / steps)
+    calls.clear()
+    assert bench.hf_cuda_sample(2, 4, 3, steps=2)["steps"] == 2 and len(calls) == 3     # the bounded block of the default native line
+
+
 def test_insitu_trace_labelling_and_durations(bench, monkeypatch):
     """bench.py's in-situ roofline: kernels of one graph-replayed decode step are labelled by order (per layer qkv, o, gate/up, down; the
     129th swap-AB GEMM is lm_head) and a kernel's duration is its successor's dependency-resolved time minus its own, so the

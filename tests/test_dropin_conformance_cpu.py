@@ -1,9 +1,10 @@
-"""Static drop-in check against the reference's OWN call sites (authoring container only: /root/reference does not travel to the GPU
-box, where tests/test_loader_gpu.py replays the same call sequence on the device instead).  Every `visualcla.<name>(...)` call in
-scripts/inference/inference.py and scripts/inference/gradio_demo.py must resolve in this package with a signature that accepts the
-keywords the script passes, and every method / attribute the scripts touch on the model object must exist on VisualCLAModel."""
-import ast
+"""Static drop-in check against the original project's OWN call sites, as recorded in tests/golden/dropin_callsites.json
+(oracle/gen_golden_dropin.py; tests/test_loader_gpu.py replays the same call sequence on the device).  Every
+`visualcla.<name>(...)` call in scripts/inference/inference.py and scripts/inference/gradio_demo.py must resolve in this
+package with a signature that accepts the keywords the script passes, and every method / attribute the scripts touch on the
+model object must exist on VisualCLAModel."""
 import inspect
+import json
 import os
 
 import pytest
@@ -11,35 +12,21 @@ import pytest
 import visualcla
 from visualcla.modeling_visualcla import VisualCLAModel, _SubModel
 
-REF = "/root/reference/scripts/inference"
 SCRIPTS = ["inference.py", "gradio_demo.py"]
 
 
-def _calls(tree, root_name):
-    """(attribute chain, keyword names, n positional) of every call whose function is an attribute chain starting at `root_name`."""
-    out = []
-    for node in ast.walk(tree):
-        if not isinstance(node, ast.Call):
-            continue
-        chain, f = [], node.func
-        while isinstance(f, ast.Attribute):
-            chain.append(f.attr)
-            f = f.value
-        if isinstance(f, ast.Call):          # e.g. model.text_model.get_input_embeddings().weight.size(0): follow the inner call too
-            continue
-        if isinstance(f, ast.Name) and f.id == root_name and chain:
-            out.append((list(reversed(chain)), [k.arg for k in node.keywords if k.arg], len(node.args)))
-    return out
+@pytest.fixture(scope="module")
+def callsites(golden_dir):
+    with open(os.path.join(golden_dir, "dropin_callsites.json")) as fh:
+        return json.load(fh)
 
 
 @pytest.mark.parametrize("script", SCRIPTS)
-def test_reference_scripts_resolve_against_this_package(script):
-    path = os.path.join(REF, script)
-    if not os.path.exists(path):
-        pytest.skip("the reference tree is only present in the authoring container")
-    tree = ast.parse(open(path).read())
+def test_reference_scripts_resolve_against_this_package(callsites, script):
+    rec = callsites["scripts"][script]
     seen = []
-    for chain, kws, npos in _calls(tree, "visualcla"):
+    for call in rec["visualcla_calls"]:
+        chain, kws, npos = call["chain"], call["keywords"], call["n_positional"]
         obj = visualcla
         for name in chain:
             assert hasattr(obj, name), f"{script}: visualcla.{'.'.join(chain)} does not exist in the drop-in package"
@@ -53,16 +40,15 @@ def test_reference_scripts_resolve_against_this_package(script):
         seen.append(".".join(chain))
     assert seen, f"{script} makes no visualcla.* call?"
     # attribute imports:  from visualcla.modeling_utils import DEFAULT_GENERATION_CONFIG  (gradio_demo.py:2)
-    for node in ast.walk(tree):
-        if isinstance(node, ast.ImportFrom) and node.module and node.module.startswith("visualcla"):
-            mod = __import__(node.module, fromlist=["x"])
-            for a in node.names:
-                assert hasattr(mod, a.name), f"{script}: from {node.module} import {a.name}"
+    for imp in rec["imports"]:
+        mod = __import__(imp["module"], fromlist=["x"])
+        for name in imp["names"]:
+            assert hasattr(mod, name), f"{script}: from {imp['module']} import {name}"
     # methods / attributes the scripts use on the model objects
-    for root in ("model", "base_model"):
-        for chain, _kws, _n in _calls(tree, root):
+    for root, chains in rec["model_calls"].items():
+        for chain in chains:
             cls = VisualCLAModel
-            for i, name in enumerate(chain):
+            for name in chain:
                 if name in ("text_model", "vision_model", "visual_resampler"):      # set per instance in __init__: handles of type _SubModel
                     cls = _SubModel
                     continue
@@ -73,15 +59,10 @@ def test_reference_scripts_resolve_against_this_package(script):
         assert "get_model_and_tokenizer_and_processor" in seen and "chat" in seen
 
 
-def test_loader_signature_matches_the_reference_definition():
-    """Same parameter names, order and defaults as ref models/visualcla/modeling_utils.py:83-92 (plus **engine_kwargs)."""
-    path = "/root/reference/models/visualcla/modeling_utils.py"
-    if not os.path.exists(path):
-        pytest.skip("the reference tree is only present in the authoring container")
-    tree = ast.parse(open(path).read())
-    ref = {n.name: n for n in ast.walk(tree) if isinstance(n, ast.FunctionDef)}
-    for fn in ("get_model_and_tokenizer_and_processor", "chat", "chat_in_stream", "encoding_text"):
-        want = [a.arg for a in ref[fn].args.args]
+def test_loader_signature_matches_the_reference_definition(callsites):
+    """Same parameter names in the same order as the original models/visualcla/modeling_utils.py:83-92 (plus **engine_kwargs)."""
+    for fn, want in callsites["loader_parameters"].items():
         have = [p.name for p in inspect.signature(getattr(visualcla.modeling_utils, fn)).parameters.values()
                 if p.kind in (p.POSITIONAL_ONLY, p.POSITIONAL_OR_KEYWORD)]
         assert have[: len(want)] == want, f"{fn}: reference parameters {want}, drop-in {have}"
+    assert set(callsites["loader_parameters"]) == {"get_model_and_tokenizer_and_processor", "chat", "chat_in_stream", "encoding_text"}
